@@ -2,6 +2,7 @@
 """bench.py -- H.x throughput of the B200-native hot path (driver contract; DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--dtype c128|f64] [--secondary a,b|none]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's algorithm on the host cores (oracle port)
 
 A "step" is one matrix-vector product y <- H x over the whole basis of the workload.  The workload is
@@ -53,6 +54,7 @@ SECONDARY = ["heisenberg_chain_24", "heisenberg_kagome_16", "heisenberg_chain_32
 X_RECIPE = "numpy RandomState(42): rand(N) - 0.5 in global sorted order (+ 1j (rand(N) - 0.5) for c128)"
 L2_NOTE = "GPU arm: 256 MB written between timed products (L2 flush); CPU arm: not applicable"
 METRIC = "H.x basis states/s"
+DUMP_ROWS, DUMP_SEED = 1 << 21, 0     # --dump-outputs: 48 MB for c128
 
 
 def parse_args():
@@ -68,6 +70,8 @@ def parse_args():
     ap.add_argument("--sample-rows", type=int, default=2048, help="rows per rank checked against the oracle")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write y of the last timed product (a fixed, seeded sample of its rows) as DIR/*.npy")
     return ap.parse_args()
 
 
@@ -394,7 +398,8 @@ class Workload:
         self.op.close()
 
 
-def time_products(w: Workload, steps: int, warmup: int, flush, barrier, dist, local_rank: int, sample_clocks: bool):
+def time_products(w: Workload, steps: int, warmup: int, flush, barrier, dist, local_rank: int, sample_clocks: bool,
+                  keep_last: bool = False):
     import torch
     from distributed_matvec_b200 import _native as nat
     for _ in range(max(warmup, 3)):
@@ -420,6 +425,9 @@ def time_products(w: Workload, steps: int, warmup: int, flush, barrier, dist, lo
     if sampler:
         sampler.__exit__()
     launches = nat.lib().dmv_launch_count() - launches0
+    if keep_last:
+        w.op.synchronize()
+        w.y_last = w.y_dev.cpu().numpy()     # before the untimed products below overwrite y
     step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     t = torch.tensor([float(np.mean(step_ms)), float(np.min(step_ms))] + step_ms, dtype=torch.float64, device="cuda")
     if w.world > 1:
@@ -443,6 +451,29 @@ def time_products(w: Workload, steps: int, warmup: int, flush, barrier, dist, lo
     if 0.0 < w.table_refill_ms < kernel_ms:
         kernel_ms -= w.table_refill_ms
     return float(t[0]), float(t[1]), kernel_ms, int(launches), (sampler.summary() if sampler else None)
+
+
+def dump_outputs(w: Workload, out_dir: str, dist):
+    """`--dump-outputs`: y of the last timed product at a fixed, seeded sample of DUMP_ROWS rows of the global sorted
+    basis (every row when the basis is smaller), so that two builds can be compared output for output.  y.npy holds
+    float64 values, shape (rows,) for f64 and (rows, 2) = (real, imag) for c128; y_rows.npy the row indices (float64)."""
+    import torch
+    n = w.n_total
+    k = min(n, DUMP_ROWS)
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=k, replace=False))
+    pos = np.minimum(np.searchsorted(rows, w.local_rows), k - 1)
+    mine = rows[pos] == w.local_rows
+    sample = np.zeros(k, dtype=w.y_last.dtype)
+    sample[pos[mine]] = w.y_last[mine]
+    if w.world > 1:      # every sampled row is owned by exactly one rank
+        t = torch.from_numpy(sample.view(np.float64)).cuda()
+        dist.all_reduce(t)
+        sample = t.cpu().numpy().view(sample.dtype)
+    if w.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        y = sample.view(np.float64)
+        np.save(os.path.join(out_dir, "y.npy"), y.reshape(k, 2) if w.cplx else y)
+        np.save(os.path.join(out_dir, "y_rows.npy"), rows.astype(np.float64))
 
 
 def roofline_of(w: Workload, kernel_ms: float, clocks: dict | None, dtype: str) -> dict:
@@ -477,6 +508,8 @@ def roofline_of(w: Workload, kernel_ms: float, clocks: dict | None, dtype: str) 
 def main():
     args = parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the product of the GPU arm; --impl reference times a slab of rows")
         run_reference(args)
         return
 
@@ -509,7 +542,9 @@ def main():
     assert n_total == w.n_total
 
     ms_per_step, ms_best, kernel_ms, launches, clocks = time_products(w, args.steps, args.warmup, flush, barrier, dist,
-                                                                     local_rank, True)
+                                                                     local_rank, True, keep_last=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(w, args.dump_outputs, dist)
 
     # ---- e2e: pinned host x -> public call -> host y; wall clock around the blocking call
     for _ in range(2):

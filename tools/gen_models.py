@@ -3,13 +3,13 @@
 
 The model inputs are data, not code: the basis description (number of spins, Hamming weight, spin
 inversion, symmetry generators) and the Hamiltonian term list (expression + site tuples) of each
-/root/reference/data/*.yaml.  This script extracts that semantic content and re-emits it in a
-normalised layout (no anchors, no comments, no solver-only keys such as `observables`,
-`number_vectors`, `output`, `max_primme_*`), so that tests, bench.py and smoke() can run on the GPU
-box where /root/reference does not exist.  tests/test_host.py (test_model_inputs_equal_the_reference_inputs) re-checks semantic equality against
-/root/reference whenever it is present.
+of the reference's data/*.yaml, kept verbatim in tests/golden/reference_models/.  This script extracts
+that semantic content and re-emits it in a normalised layout (no anchors, no comments, no solver-only
+keys such as `observables`, `number_vectors`, `output`, `max_primme_*`), the one tests, bench.py and
+smoke() read.  tests/test_host.py (test_model_inputs_equal_the_reference_inputs) re-checks semantic
+equality against tests/golden/reference_models/.
 
-Usage:  python tools/gen_models.py [/root/reference/data] [data]
+Usage:  python tools/gen_models.py [tests/golden/reference_models] [data]
 """
 import glob
 import os
@@ -53,8 +53,9 @@ def normalise(conf: dict) -> dict:
 
 
 def main():
-    src = sys.argv[1] if len(sys.argv) > 1 else "/root/reference/data"
-    dst = sys.argv[2] if len(sys.argv) > 2 else os.path.join(os.path.dirname(__file__), "..", "data")
+    root = os.path.join(os.path.dirname(__file__), "..")
+    src = sys.argv[1] if len(sys.argv) > 1 else os.path.join(root, "tests", "golden", "reference_models")
+    dst = sys.argv[2] if len(sys.argv) > 2 else os.path.join(root, "data")
     os.makedirs(dst, exist_ok=True)
     for path in sorted(glob.glob(os.path.join(src, "*.yaml"))):
         with open(path, "r", encoding="utf-8") as f:
