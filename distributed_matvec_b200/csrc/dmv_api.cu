@@ -642,6 +642,7 @@ void ensure_table(dmv_context *ctx, int elt) {
   CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
   int64_t per_state = ce ? 8 : 2;
   while (per_state > 2 && (double)per_state * n_left * 32.0 > 0.25 * (double)free_b) per_state /= 2;
+  if (ce && ctx->opt_table_per_state > 0) per_state = ctx->opt_table_per_state;
   if (per_state * n_left + 16 >= 2147483647ll) throw std::runtime_error("k_rows: table of more than 2^31 buckets");
   const uint32_t slots = (uint32_t)std::max<int64_t>(16, per_state * n_left);
   ctx->d_table.alloc((size_t)slots * 32);
@@ -684,7 +685,8 @@ void rows_product(dmv_context *basis, KernelParams &p, int elt, const void *x_al
   p.mph = basis->mph;
   p.dense = basis->dense_index ? basis->d_dense.ptr : nullptr;
   p.row_split = 1;
-  launch_rows(p, elt == DMV_C128, stream);
+  const int launched = launch_rows(p, elt == DMV_C128, stream);
+  if (launched) basis->rows_kernel = timer->rows_kernel = launched;
 }
 
 // the same for `nv` vectors at once (single rank; x / y: nv device vectors `stride` elements apart): k_rows_batch
@@ -699,6 +701,7 @@ void rows_product_batch(dmv_context *ctx, int elt, int nv, const void *x, void *
     CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
     int64_t per_state = 8;
     while (per_state > 2 && (double)per_state * n * 64.0 > 0.25 * (double)free_b) per_state /= 2;
+    if (ctx->opt_table_per_state > 0) per_state = ctx->opt_table_per_state;
     if (per_state * n + 16 >= 2147483647ll) throw std::runtime_error("k_rows_batch: table of more than 2^31 buckets");
     const uint32_t buckets = (uint32_t)std::max<int64_t>(16, per_state * n);
     ctx->d_table_batch.alloc((size_t)buckets * 64);
@@ -720,7 +723,8 @@ void rows_product_batch(dmv_context *ctx, int elt, int nv, const void *x, void *
   p.batch_elt = elt;
   p.batch_stride = stride;
   p.row_split = 1;
-  launch_rows_batch(p, st);
+  const int launched = launch_rows_batch(p, st);
+  if (launched) ctx->rows_batch_kernel = launched;
 }
 
 void do_generate(dmv_context *ctx, int elt, const void *x_dev, void *y_dev,
@@ -1005,8 +1009,15 @@ int dmv_set_option(dmv_context *ctx, const char *name, int64_t value) {
     if (value < -1 || value > 0) throw std::runtime_error("gather: -1 auto, 0 off (queued k_pull for mode = 1)");
     ctx->opt_gather = (int)value;
   } else if (key == "rows_batch_min") {
-    if (value < 2 || value > 6) throw std::runtime_error("rows_batch_min: 2 .. 6 doubles per state");
+    if (value < 1 || value > 6) throw std::runtime_error("rows_batch_min: 1 .. 6 doubles per state");
     ctx->opt_rows_batch_min = (int)value;
+  } else if (key == "rows_table_per_state") {
+    if (value != 0 && value != 2 && value != 4 && value != 8)
+      throw std::runtime_error("rows_table_per_state: 0 auto, or 2 / 4 / 8 buckets per state");
+    ctx->opt_table_per_state = (int)value;
+    ctx->table_elt = 0;
+    ctx->table_batch_slots = 0;
+    if (ctx->global) { ctx->global->opt_table_per_state = (int)value; ctx->global->table_elt = 0; }
   } else if (key == "rows_batch") {
     if (value < -1 || value > 1) throw std::runtime_error("rows_batch: -1 auto / 1 k_rows_batch for batched products, 0 vector by vector");
     ctx->opt_rows_batch = (int)value;
@@ -1069,6 +1080,10 @@ int64_t dmv_get_info(const dmv_context *ctx, const char *name) {
     return ((use_pull(ctx) && !use_gather(ctx) && use_rows(ctx)) ||
             (ctx->replicated && ctx->global && !use_gather(ctx->global) && use_rows(ctx->global))) ? 1 : 0;
   if (key == "rows_ok") return ctx->rows_ok ? 1 : 0;
+  if (key == "rows_kernel") return ctx->rows_kernel;
+  if (key == "rows_batch_kernel") return ctx->rows_batch_kernel;
+  if (key == "rows_table_buckets") return (int64_t)ctx->table_slots;
+  if (key == "rows_batch_buckets") return (int64_t)ctx->table_batch_slots;
   if (key == "rows_dense") return ctx->dense_index ? (int64_t)ctx->mph.n_dense : (ctx->global && ctx->global->dense_index ? (int64_t)ctx->global->mph.n_dense : 0);
   if (key == "rounds") return ctx->rounds.ready ? ctx->rounds.R : 0;
   if (key == "peer_gather") return (ctx->replicated && ctx->peer_gather) ? 1 : 0;
@@ -1248,7 +1263,7 @@ int dmv_generate(dmv_context *ctx, int elt, const void *x, void *y) {
   use_device(ctx);
   require_states(ctx);
   if (elt != DMV_F64 && elt != DMV_C128) throw std::runtime_error("elt must be DMV_F64 or DMV_C128");
-  if (!is_device_pointer(x) || !is_device_pointer(y))
+  if (!is_device_vector(x, ctx->n_states) || !is_device_vector(y, ctx->n_states))
     throw std::runtime_error("dmv_generate needs device pointers (y is accumulated into by later steps)");
   do_generate(ctx, elt, x, y);
   check_status(ctx);
@@ -1270,7 +1285,7 @@ int dmv_accumulate(dmv_context *ctx, int elt, int64_t count, const uint64_t *bet
   API_BEGIN
   use_device(ctx);
   require_states(ctx);
-  if (!is_device_pointer(y)) throw std::runtime_error("dmv_accumulate needs a device y");
+  if (!is_device_vector(y, ctx->n_states)) throw std::runtime_error("dmv_accumulate needs a device y");
   const int width = complex_values(ctx, elt) ? 2 : 1;
   InArg<uint64_t> b(betas, (size_t)count, ctx->stream);
   InArg<double> c(coeffs, (size_t)count * width, ctx->stream);
@@ -1362,7 +1377,8 @@ int dmv_matvec_batch(dmv_context *ctx, int elt, int num_vectors, const void *x, 
     const bool on_host = !is_device_pointer(x);
     // (a batch costs 1.5 - 1.6 single products on the 6x6 square -- 64-byte buckets, one request per lane in flight:
     // profiles/r02_rows_batch_6x6.md -- so it pays from two vectors on)
-    while ((num_vectors - k) * elt >= ctx->opt_rows_batch_min && num_vectors - k >= 2) {
+    // (rows_batch_min = 1 sends a single vector through k_rows_batch as well)
+    while ((num_vectors - k) * elt >= ctx->opt_rows_batch_min && num_vectors - k >= std::min(2, ctx->opt_rows_batch_min)) {
       const int nv = std::min(per, num_vectors - k);
       const void *xk = xb + (size_t)k * vec_bytes;
       void *yk = yb + (size_t)k * vec_bytes;

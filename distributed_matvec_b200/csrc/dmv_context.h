@@ -78,6 +78,9 @@ inline bool is_device_pointer(const void *p) {
   if (e != cudaSuccess) { cudaGetLastError(); return false; }
   return attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged;
 }
+// a vector of a context that owns no states (a rank of a small basis) has no elements: a tensor of zero elements may
+// carry a null pointer, and nothing is read from or written to it
+inline bool is_device_vector(const void *p, int64_t n_states) { return n_states == 0 ? true : is_device_pointer(p); }
 
 // ---- NCCL through dlopen ------------------------------------------------------------------------
 struct NcclApi {
@@ -192,6 +195,9 @@ struct dmv_context {
   bool rows_ok = false;
   int opt_rows = -1;        // -1 auto (k_rows when it applies), 0 the queued k_pull
   int opt_rows_ctas = 3;    // k_rows: resident CTAs per SM: 3 (80 registers, default) | 2 (122 registers) | 4 (64 registers)
+  int rows_kernel = 0;      // instantiation of the last k_rows launch: 100 CTAS + 10 TK + MPH (0: none yet)
+  int rows_batch_kernel = 0;   // the same for k_rows_batch: 100 CTAS + 10 TK
+  int opt_table_per_state = 0;   // buckets per state of the complex128 and k_rows_batch tables: 0 auto | 2 | 4 | 8
   int opt_gather_walk = 0;  // k_gather: 0 per-lane walk from the top bit (default), 1 group-major warp-uniform walk
                             // (measured slower), 2 per-lane walk from the bottom bit (round 1)
   DevBuf<unsigned char> d_table;

@@ -127,6 +127,7 @@ void setup_replicated(dmv_context *ctx) {
     g->opt_gather_walk = ctx->opt_gather_walk;
     g->opt_rows_index = ctx->opt_rows_index;
     g->opt_rows_ctas = ctx->opt_rows_ctas;
+    g->opt_table_per_state = ctx->opt_table_per_state;
     if (ctx->opt_canon != g->opt_canon && g->proj == PROJ_GROUP) { g->opt_canon = ctx->opt_canon; upload_orbit(g); }
     if (dmv_basis_build(g) != 0) throw std::runtime_error(g_last_error);
   }
@@ -846,7 +847,7 @@ int dmv_replicated_product(dmv_context *ctx, int elt, const void *x_cat, void *y
   require_states(ctx);
   if (!ctx->global || ctx->repl_block <= 0) throw std::runtime_error("dmv_replicated_setup has not run");
   if (elt != DMV_F64 && elt != DMV_C128) throw std::runtime_error("elt must be DMV_F64 or DMV_C128");
-  if (!is_device_pointer(x_cat) || !is_device_pointer(y)) throw std::runtime_error("dmv_replicated_product needs device pointers");
+  if (!is_device_pointer(x_cat) || !is_device_vector(y, ctx->n_states)) throw std::runtime_error("dmv_replicated_product needs device pointers");
   replicated_rows(ctx, elt, x_cat, y);
   check_status(ctx);
   API_END

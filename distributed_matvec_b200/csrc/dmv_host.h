@@ -125,14 +125,15 @@ void launch_pull(const KernelParams &p, Projection proj, bool complex_values, bo
 // row traversal without queue / atomics for bit-parallel operators on unprojected or inversion-only bases
 void launch_gather(const KernelParams &p, bool inversion, bool complex_values, bool complex_elements,
                    bool narrow, bool lin, bool uniform, cudaStream_t stream);
-// k_rows applies to real operators with a bit-parallel emit test on bases with trivial characters
-void launch_rows(const KernelParams &p, bool complex_elements, cudaStream_t stream);
+// k_rows applies to real operators with a bit-parallel emit test on bases with trivial characters; returns the
+// instantiation it launched as 100 CTAS + 10 TK + MPH (0: nothing launched)
+int launch_rows(const KernelParams &p, bool complex_elements, cudaStream_t stream);
 // hash table of k_rows: insert every state (slot_of[i] = its slot), then per product table[slot_of[i]] = x[src(i)] * norm[i]
 // with src(i) = pos ? pos[i] : i
 void launch_table_insert(const uint64_t *reps, int64_t n, void *table, uint32_t n_buckets, int slots_per_bucket,
                          uint32_t *slot_of, cudaStream_t stream, int bucket_bytes = 32);
 // k_rows on several vectors at once: 64-byte buckets { key, six doubles, spare } shared by the vectors of the batch
-void launch_rows_batch(const KernelParams &p, cudaStream_t stream);
+int launch_rows_batch(const KernelParams &p, cudaStream_t stream);   // -> 100 CTAS + 10 TK (0: nothing launched)
 void launch_table_fill_batch(int64_t n, int num_vectors, int elt, const void *x, int64_t stride, const double *norms,
                              const uint32_t *slot_of, const uint64_t *reps, void *table, cudaStream_t stream);
 void launch_table_fill(int64_t n, bool complex_elements, const void *x, const double *norms, const uint32_t *pos,

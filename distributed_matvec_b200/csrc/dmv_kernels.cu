@@ -1611,7 +1611,7 @@ void launch_accumulate_p(const KernelParams &p, bool cv, bool ce, int64_t count,
 
 namespace {
 template <bool CE, int TK, bool MPH, int CTAS = 2>
-void launch_rows_t(const KernelParams &p, cudaStream_t stream) {
+int launch_rows_t(const KernelParams &p, cudaStream_t stream) {
   const SmemLayout L = smem_layout(p, PROJ_GROUP, sizeof(double), false);
   const size_t smem_bytes = L.total;
   auto kernel = k_rows<CE, TK, MPH, CTAS>;
@@ -1625,39 +1625,37 @@ void launch_rows_t(const KernelParams &p, cudaStream_t stream) {
   kernel<<<blocks, kThreads, smem_bytes, stream>>>(p);
   DMV_CUDA_CHECK(cudaGetLastError());
   g_launches++;
+  return 100 * CTAS + 10 * TK + (MPH ? 1 : 0);
 }
 template <bool CE>
-void launch_rows_e(const KernelParams &p, cudaStream_t stream) {
+int launch_rows_e(const KernelParams &p, cudaStream_t stream) {
   const OrbitProgram &o = p.orbit;
   const int k = (o.canon_mode != 0 && o.tor_mode == 2 && o.canon_k == o.canon_r) ? o.canon_k : 0;
   if (p.dense != nullptr) {   // dense index (perfect hash)
-    if (k == 6) launch_rows_t<CE, 6, true>(p, stream);
-    else if (k == 4) launch_rows_t<CE, 4, true>(p, stream);
-    else launch_rows_t<CE, 0, true>(p, stream);
-    return;
+    if (k == 6) return launch_rows_t<CE, 6, true>(p, stream);
+    if (k == 4) return launch_rows_t<CE, 4, true>(p, stream);
+    return launch_rows_t<CE, 0, true>(p, stream);
   }
   if (p.rows_ctas == 2) {   // two CTAs per SM: 122 registers, nothing spills
-    if (k == 6) launch_rows_t<CE, 6, false>(p, stream);
-    else if (k == 4) launch_rows_t<CE, 4, false>(p, stream);
-    else launch_rows_t<CE, 0, false>(p, stream);
-    return;
+    if (k == 6) return launch_rows_t<CE, 6, false>(p, stream);
+    if (k == 4) return launch_rows_t<CE, 4, false>(p, stream);
+    return launch_rows_t<CE, 0, false>(p, stream);
   }
   if (p.rows_ctas == 4) {   // four CTAs per SM: 64 registers
-    if (k == 6) launch_rows_t<CE, 6, false, 4>(p, stream);
-    else launch_rows_t<CE, 0, false, 4>(p, stream);
-    return;
+    if (k == 6) return launch_rows_t<CE, 6, false, 4>(p, stream);
+    return launch_rows_t<CE, 0, false, 4>(p, stream);
   }
   // default: three CTAs per SM (80 registers; a few words of the pipeline state spill, 24 warps per SM more than pay for it:
   // 6x6 24.9 -> 22.3 ms, chain_36_symm 53.5 -> 44.0 ms, profiles/r02_rows_pipelines.md)
-  if (k == 6) launch_rows_t<CE, 6, false, 3>(p, stream);
-  else if (k == 4) launch_rows_t<CE, 4, false, 3>(p, stream);
-  else launch_rows_t<CE, 0, false, 3>(p, stream);
+  if (k == 6) return launch_rows_t<CE, 6, false, 3>(p, stream);
+  if (k == 4) return launch_rows_t<CE, 4, false, 3>(p, stream);
+  return launch_rows_t<CE, 0, false, 3>(p, stream);
 }
 }  // namespace
 
 namespace {
 template <int TK, int CTAS>
-void launch_rows_batch_t(const KernelParams &p, cudaStream_t stream) {
+int launch_rows_batch_t(const KernelParams &p, cudaStream_t stream) {
   const SmemLayout L = smem_layout(p, PROJ_GROUP, sizeof(double), false);
   const size_t smem_bytes = L.total;
   auto kernel = k_rows_batch<TK, CTAS>;
@@ -1671,21 +1669,22 @@ void launch_rows_batch_t(const KernelParams &p, cudaStream_t stream) {
   kernel<<<blocks, kThreads, smem_bytes, stream>>>(p);
   DMV_CUDA_CHECK(cudaGetLastError());
   g_launches++;
+  return 100 * CTAS + 10 * TK;
 }
 }  // namespace
 
 // p.batch vectors of p.batch_elt doubles per element (p.batch * p.batch_elt <= 6), p.table = the 64-byte-bucket table
-void launch_rows_batch(const KernelParams &p, cudaStream_t stream) {
-  if (p.row_end <= p.row_begin) return;
+int launch_rows_batch(const KernelParams &p, cudaStream_t stream) {
+  if (p.row_end <= p.row_begin) return 0;
   if (p.batch < 1 || (p.batch_elt != 1 && p.batch_elt != 2) || p.batch * p.batch_elt > 6)
     throw std::runtime_error("k_rows_batch: at most six doubles per state");
   const OrbitProgram &o = p.orbit;
   const int k = (o.canon_mode != 0 && o.tor_mode == 2 && o.canon_k == o.canon_r) ? o.canon_k : 0;
   // two CTAs per SM (120-128 registers: the eight words of the request stay in registers; at 80 registers part of them
   // spills and the batch is 4 % slower: profiles/r02_rows_batch_6x6.md)
-  if (k == 6) launch_rows_batch_t<6, 2>(p, stream);
-  else if (k == 4) launch_rows_batch_t<4, 2>(p, stream);
-  else launch_rows_batch_t<0, 2>(p, stream);
+  if (k == 6) return launch_rows_batch_t<6, 2>(p, stream);
+  if (k == 4) return launch_rows_batch_t<4, 2>(p, stream);
+  return launch_rows_batch_t<0, 2>(p, stream);
 }
 
 void launch_table_fill_batch(int64_t n, int num_vectors, int elt, const void *x, int64_t stride, const double *norms,
@@ -1698,10 +1697,9 @@ void launch_table_fill_batch(int64_t n, int num_vectors, int elt, const void *x,
   g_launches++;
 }
 
-void launch_rows(const KernelParams &p, bool complex_elements, cudaStream_t stream) {
-  if (p.row_end <= p.row_begin) return;
-  if (complex_elements) launch_rows_e<true>(p, stream);
-  else launch_rows_e<false>(p, stream);
+int launch_rows(const KernelParams &p, bool complex_elements, cudaStream_t stream) {
+  if (p.row_end <= p.row_begin) return 0;
+  return complex_elements ? launch_rows_e<true>(p, stream) : launch_rows_e<false>(p, stream);
 }
 
 void launch_table_insert(const uint64_t *reps, int64_t n, void *table, uint32_t n_buckets, int slots_per_bucket,

@@ -86,6 +86,10 @@ int dmv_synchronize(dmv_context *ctx);
  *          "rows_batch" = -1 auto, 1: dmv_matvec_batch on bases with permutation symmetries takes up to six doubles per
  *                        state (six real / three complex vectors) through k_rows_batch | 0 vector by vector;
  *                        "rows_batch_min" = doubles per state (vectors x element width, default 2) from which it is used
+ *                        (1: a single real vector goes through k_rows_batch too)
+ *          "rows_table_per_state" = 0 auto (complex128 k_rows table and k_rows_batch table: 8 buckets per state, 4 or 2
+ *                        when the table would take more than a quarter of the free memory) | 2 | 4 | 8 forced; the
+ *                        float64 k_rows table always has 2 two-slot buckets per state
  *          "gather_walk" = 0 every lane walks its emitting groups from the top bit | 1 group-major warp-uniform walk
  *                        (measured slower) | 2 from the bottom bit (round 1)
  *          "index"    = -1 auto (identity / Lin tables / directory) | 0 directory + binary search | 2 combinadic rank
@@ -101,7 +105,11 @@ int dmv_synchronize(dmv_context *ctx);
  *                        (generate everything, fence, accumulate) | R <= 64 rounds
  * dmv_get_info: "index_mode", "pull", "gather", "rows", "rows_ok", "projection", "n_groups", "orbit_n_q", "orbit_n_t",
  *               "canon_mode", "torus_mode", "peer_direct", "replicated", "replicated_block", "peer_gather", "rounds",
- *               "global_states", "complex_coefficients", ... (-1: unknown) */
+ *               "global_states", "complex_coefficients", "rows_kernel" (instantiation of the last k_rows launch:
+ *               100 CTAS + 10 TK + MPH, CTAS = resident CTAs per SM, TK = torus block size of the canonical form or 0,
+ *               MPH = 1 with the dense index; 0 before the first launch), "rows_batch_kernel" (the same for the last
+ *               k_rows_batch launch), "rows_table_buckets" / "rows_batch_buckets" (buckets of the k_rows / k_rows_batch
+ *               open-addressing table as last built; 0 before), ... (-1: unknown) */
 int dmv_set_option(dmv_context *ctx, const char *name, int64_t value);
 int64_t dmv_get_info(const dmv_context *ctx, const char *name);
 
